@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the headline benchmark (BASELINE.json: uncompressed GB/s, level-3 compress + decompress).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--chunks C] [--level L]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--chunks C] [--level L] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 A *step* is one pass of the hot path over one batch: every rank compresses its shard of C 128 KB chunks
@@ -179,6 +179,7 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the sub-records (levels, configs[3], configs[4])")
     ap.add_argument("--strong", action="store_true", help="also run the strong-scaling data-plane record at N = 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed on rank 0 to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     from zstd_jni_b200 import corpus
@@ -295,6 +296,8 @@ def main():
         launches = ctx.kernelLaunches() - launches0
         ktimes = ctx.kernelTimes()
         clocks = sampler.stop()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(Path(args.dump_outputs), n, d_sizes, d_ooff, d_out, d_back, d_res)
         # The entropy stage runs beside the parse (one timed entry, "k_parse+k_entropy"); a short pass with the two serialized gives the
         # stage times on their own -- reported as such, not part of the timed region.
         ctx.setOption("entropy_overlap", 0)
@@ -337,7 +340,7 @@ def main():
         de(K - 1)
         torch.cuda.synchronize()
     e2e_run(2); barrier()
-    e2e_steps = max(4, min(args.steps, 32))          # the pipeline fills and drains once per run (~60 ms that no step can hide): the K steps asked for, at least 4
+    e2e_steps = args.steps                           # the pipeline fills and drains once per run (~60 ms that no step can hide)
     t0 = time.perf_counter()
     e2e_run(e2e_steps)
     e2e_s = (time.perf_counter() - t0) / e2e_steps
@@ -433,6 +436,22 @@ def main():
     print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir: Path, n, d_sizes, d_ooff, d_out, d_back, d_res):
+    """What a caller of the timed path receives, as float arrays (bytes and sizes are exact in them), so that two builds can be compared
+    output for output: every frame size and regenerated size, and for a fixed, seeded sample of 32 chunks their frames and regenerated
+    bytes (about 25 MB for the default workload, at most 34 MB; the whole round trip is checked on the device by the run itself)."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    offs = d_ooff.cpu().numpy()
+    pick = np.sort(np.random.default_rng(0).choice(n, size=min(n, 32), replace=False))
+    frames = np.concatenate([d_out[offs[i]:offs[i + 1]].cpu().numpy() for i in pick])
+    back = np.concatenate([d_back[i * CHUNK:(i + 1) * CHUNK].cpu().numpy() for i in pick])
+    np.save(out_dir / "frame_sizes.npy", d_sizes.cpu().numpy().astype(np.float64))
+    np.save(out_dir / "decompressed_sizes.npy", d_res.cpu().numpy().astype(np.float64))
+    np.save(out_dir / "sample_chunks.npy", pick.astype(np.float64))
+    np.save(out_dir / "sample_frames.npy", frames.astype(np.float32))
+    np.save(out_dir / "sample_decompressed.npy", back.astype(np.float32))
 
 
 # ----------------------------------------------------------------------------- sub-records

@@ -18,13 +18,3 @@ def _built():
     import __graft_entry__ as g
     g.build()
     yield
-
-
-REFERENCE_RESOURCES = Path("/root/reference/src/test/resources")
-
-
-@pytest.fixture(scope="session")
-def reference_resources():
-    if not REFERENCE_RESOURCES.exists():
-        pytest.skip("reference test resources not present on this machine")
-    return REFERENCE_RESOURCES

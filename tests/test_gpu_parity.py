@@ -10,7 +10,8 @@ import numpy as np
 import pytest
 
 from tests import cases
-from tests.oracle_util import oracle_compress, oracle_decompress, ref, ref_compress, ref_stream_compress
+from tests.golden.make_golden_xml import SAMPLE, is_xml_sample, xml_frame
+from tests.oracle_util import oracle_compress, oracle_decompress, ref_compress
 
 pytestmark = pytest.mark.gpu
 GOLDEN = Path(__file__).parent / "golden"
@@ -26,8 +27,7 @@ def ctx():
 
 def _expected(data, level):
     r = oracle_compress(data, level)
-    if ref() is not None:
-        assert ref_compress(data, level) == r
+    assert ref_compress(data, level) == r
     return r
 
 
@@ -110,7 +110,6 @@ def _literal_payload(z: bytes):
     return blk + lh, blk + lh + csz
 
 
-@pytest.mark.skipif(ref() is None, reason="oracle/_ref not built")
 def test_decoder_matches_the_compiled_reference_on_corruptions(ctx):
     """The same single-bit corruptions judged by the reference itself (oracle/_ref), not by the restatement.  One class of input is
     allowed to differ, exactly as DESIGN.md section 5 documents it: a flipped bit INSIDE the compressed-literals payload, where this
@@ -123,7 +122,8 @@ def test_decoder_matches_the_compiled_reference_on_corruptions(ctx):
     for idx in (0, 1, 2, 3, 4, 5, 7, 9):
         data = corpus.chunk(idx)[:60000].tobytes()
         for level in (3, 1):
-            z = ref_compress(data, level)
+            z = oracle_compress(data, level)
+            assert z == ref_compress(data, level), (idx, level)
             lit = _literal_payload(z)
             for _ in range(40):
                 zz = bytearray(z)
@@ -143,20 +143,17 @@ def test_decoder_matches_the_compiled_reference_on_corruptions(ctx):
     assert allowed <= len(blobs) // 4 and header <= len(blobs) // 50, (allowed, header)        # minorities (~8 % and < 1 % of random flips)
 
 
-@pytest.mark.skipif(ref() is None, reason="oracle/_ref not built")
 def test_decodes_reference_streams(ctx):
-    from zstd_jni_b200 import corpus
-    data = b"".join(corpus.chunk(i).tobytes() for i in (0, 9, 2, 3, 4, 5))[:700000]
-    blobs = [ref_stream_compress(data, lv, checksum=cs) for lv in (1, 3, 9, 15) for cs in (False, True)]
-    outs = ctx.decompressBatch(blobs, [len(data)] * len(blobs))
-    assert all(o == data for o in outs)
+    """The reference's streaming path over the 256 KB sample of `xml` (tests/golden/xml), with and without checksums."""
+    blobs = [xml_frame(f"xml-{lv}{'-xxh' if cs else ''}.zst") for lv in (1, 3, 9, 15) for cs in (False, True)]
+    outs = ctx.decompressBatch(blobs, [SAMPLE] * len(blobs))
+    assert all(is_xml_sample(o) for o in outs)
 
 
-def test_reference_golden_resources(ctx, reference_resources):
-    xml = (reference_resources / "xml").read_bytes()
+def test_reference_golden_resources(ctx):
     names = ["xml-1.zst", "xml-3.zst", "xml-6.zst", "xml-9.zst", "xml-1-sized.zst"]
-    outs = ctx.decompressBatch([(reference_resources / n).read_bytes() for n in names], [len(xml)] * len(names))
-    assert all(o == xml for o in outs)
+    outs = ctx.decompressBatch([xml_frame(n) for n in names], [SAMPLE] * len(names))
+    assert all(is_xml_sample(o) for o in outs)
 
 
 def test_full_size_config_properties(ctx):
